@@ -64,6 +64,12 @@ REF_LIB = os.path.join(ORACLE_DIR, "_ref", "libref_ba.so")
 DROPIN_LIB = os.path.join(ORACLE_DIR, "_ref", "libdropin_ba.so")
 
 
+def reference_golden():
+    """What the reference's own translation units (libref_ba.so) computed on the cases of the tests that compare with the reference:
+    tests/golden/reference_small.npz, written by `python tests/golden/make_golden.py --reference`."""
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_small.npz"))
+
+
 def ref_lib(path=None):
     """oracle/_ref/libref_ba.so: the reference's own back-end translation units behind a C interface (oracle/ref_pin/ref_bench.cc).
     Built by `make -C oracle ref_pin` where /root/reference is mounted; None where it is not there (the built file travels).

@@ -14,6 +14,7 @@ import pytest
 
 from ldso_b200 import synth
 from tests import oracle_py
+from tests.golden import make_golden
 from tests.parity import rel_err
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "ba_small.npz")
@@ -293,10 +294,12 @@ def test_trace_immature_oracle():
     assert np.all(st3[oob] == oracle_py.IPS_OOB)
 
 
-REFERENCE = "/root/reference"
+PIN_DIR = os.path.join(oracle_py.ORACLE_DIR, "_ref")
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "include", "internal")), reason="the reference tree is only mounted in the build container")
+@pytest.mark.skipif(not all(os.path.exists(os.path.join(PIN_DIR, n)) for n in ("pin_ref", "pin_ref_break")),
+                    reason="oracle/_ref/pin_ref compiles an LDSO source tree's own sources (build() makes it where the tree is present; "
+                           "make -C oracle ref_pin REF=<tree>)")
 def test_oracle_pinned_against_reference_sources():
     """oracle/ref_pin: the reference's OWN Residuals.cc (linearize, applyRes/takeData, fixLinearizationF), AccumulatedTopHessian.cc /
     AccumulatedSCHessian.cc (addPoint<0,1,2>, SC addPoint, the stitchers), EnergyFunctional.cc (insertFrame, setAdjointsF, setDeltaF,
@@ -305,13 +308,12 @@ def test_oracle_pinned_against_reference_sources():
     traceOn, linearizeResidual), MatrixAccumulators.h, GlobalFuncs.h, ResidualProjections.h, AffLight.h and Setting.cc, compiled
     unmodified where they lie (against oracle/ref_shim: stand-ins for Eigen / Sophus / Frame.h / OpenCV / glog), agree bit for bit
     with the oracle on 108 checks; the negative controls (an operand scaled by 1 + 2e-7, two results moved by one ulp on the oracle
-    side) are detected."""
+    side) are detected. The two programs are the ones build() made (the reference's sources are needed to compile them, not to
+    run them)."""
     import subprocess
-    odir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle")
-    subprocess.check_call(["make", "-C", odir, "-s", "ref_pin", "REF=" + REFERENCE])
-    r = subprocess.run([os.path.join(odir, "_ref", "pin_ref")], capture_output=True, text=True)
+    r = subprocess.run([os.path.join(PIN_DIR, "pin_ref")], capture_output=True, text=True)
     assert r.returncode == 0 and "PIN OK" in r.stdout, r.stdout + r.stderr
-    r = subprocess.run([os.path.join(odir, "_ref", "pin_ref_break")], capture_output=True, text=True)
+    r = subprocess.run([os.path.join(PIN_DIR, "pin_ref_break")], capture_output=True, text=True)
     assert r.returncode != 0 and "PIN MISMATCH" in r.stdout
 
 
@@ -344,41 +346,39 @@ def test_select_activation_oracle():
     assert prev > 0
 
 
-@pytest.mark.skipif(oracle_py.ref_lib() is None, reason="oracle/_ref/libref_ba.so is built only where the reference tree is mounted (make -C oracle ref_pin)")
 def test_reference_arm_matches_oracle():
     """bench.py's reference arm (oracle/_ref/libref_ba.so: the reference's own back-end translation units + a restated FullSystem driver
     loop, built with -O3 -march=native) walks the same Gauss-Newton trajectory as the oracle port on the same window: energies, the
-    step-size criterion and the final inverse depths agree up to the FMA-contraction noise of the two optimised builds."""
-    win = synth.make_window(nF=5, pts_per_frame=60, w=320, h=240, seed=3)
-    r = oracle_py.RefBA(win, multithreaded=False)
+    step-size criterion and the final inverse depths agree up to the FMA-contraction noise of the two optimised builds. The reference's
+    side is stored in tests/golden/reference_small.npz."""
+    g = oracle_py.reference_golden()
+    win = make_golden.ref_window("small")
     o = oracle_py.OracleBA(win, threads_mode=1, fast=True)
-    e_r, e_o = r.optimize_begin(), o.optimize_begin()
+    e_r, e_o = g["small_energy"][0], o.optimize_begin()
     assert abs(e_r - e_o) <= 1e-6 * e_o
     for it in range(4):
-        br, bo = r.gn_iteration(it), o.gn_iteration(it)
-        assert br == bo
-        assert abs(r.energy() - o.energy()) <= 2e-3 * r.energy()
-    d = np.abs(r.idepths() - o.points()["idepth"])
+        assert g["small_converged"][it] == o.gn_iteration(it)
+        e_r = g["small_energy"][it + 1]
+        assert abs(e_r - o.energy()) <= 2e-3 * e_r
+    d = np.abs(g["small_idepth"][3] - o.points()["idepth"])
     assert np.median(d) < 3e-4 and d.max() < 5e-3          # the scale gauge is only damped (DESIGN section 5): a common drift of a few 1e-5
     # and with the reference's 6 worker threads (chunk sums arrive in thread order: compare loosely)
-    r6 = oracle_py.RefBA(win, multithreaded=True)
-    assert abs(r6.optimize_begin() - e_o) <= 1e-5 * e_o
-    r6.gn_iteration(0)
-    assert np.isfinite(r6.energy()) and r6.energy() < e_o
+    e6 = g["small_6threads_energy"]
+    assert abs(e6[0] - e_o) <= 1e-5 * e_o
+    assert np.isfinite(e6[1]) and e6[1] < e_o
 
 
-@pytest.mark.skipif(oracle_py.ref_lib() is None, reason="oracle/_ref/libref_ba.so is built only where the reference tree is mounted (make -C oracle ref_pin)")
 def test_reference_lastx_noise_floor_is_along_the_gauge():
     """Why parity on lastX is measured on the gauge-orthogonal complement: the reference's OWN library (its EnergyFunctional.cc, its
     accumulators, the stand-in Eigen's LDLT) and the oracle (same pinned H and b, Eigen's LDLT restated) give update vectors that differ
     by ~2e-3 as they stand -- twenty times the 1e-4 bar -- and by ~1e-5 once the seven gauge directions are projected out
     (measured: 1.6e-3 / 6.3e-6 on this window, 2.1e-3 / 1.2e-5 on the 8 x 2000-point window). Its 6-thread runs reproduced the
     1-thread bits in 5 of 5 runs on this host (the chunk scheduler hands one worker nearly everything), so the thread order is not
-    the larger effect here; the factorisation's rounding along the barely-damped scale direction is."""
-    win = synth.make_window(nF=6, pts_per_frame=120, w=320, h=240, seed=17)
-    r = oracle_py.RefBA(win, multithreaded=False)
-    r.optimize_begin(); r.gn_iteration(0)
-    xr = r.last_x()
+    the larger effect here; the factorisation's rounding along the barely-damped scale direction is. The reference's update vectors
+    are stored in tests/golden/reference_small.npz."""
+    g = oracle_py.reference_golden()
+    win = make_golden.ref_window("gauge")
+    xr = g["gauge_lastX0"]
     o = oracle_py.OracleBA(win, threads_mode=0)
     o.optimize_begin(); o.solve_system(0)
     xo = o.system()["lastX"]
@@ -387,63 +387,58 @@ def test_reference_lastx_noise_floor_is_along_the_gauge():
     raw, proj = rel_err(xo, xr), rel_err((I - P) @ xo, (I - P) @ xr)
     assert proj < 1e-4, proj
     assert proj < 0.1 * raw or raw < 1e-5, (raw, proj)          # the disagreement lives in the gauge directions
-    r6 = oracle_py.RefBA(win, multithreaded=True)
-    r6.optimize_begin(); r6.gn_iteration(0)
-    assert rel_err((I - P) @ r6.last_x(), (I - P) @ xr) < 1e-4
+    assert rel_err((I - P) @ g["gauge_6threads_lastX0"], (I - P) @ xr) < 1e-4
 
 
-@pytest.mark.skipif(oracle_py.ref_lib() is None or not os.path.exists(oracle_py.DROPIN_LIB),
-                    reason="oracle/_ref/libref_ba.so / libdropin_ba.so are built only where the reference tree is mounted (make -C oracle ref_pin dropin)")
-@pytest.mark.parametrize("drop_target,remove_every", [(-1, 0), (1, 7), (4, 3)])
+needs_dropin = pytest.mark.skipif(not os.path.exists(oracle_py.DROPIN_LIB),
+                                  reason="oracle/_ref/libdropin_ba.so compiles against an LDSO source tree's headers (make -C oracle ref_pin dropin REF=<tree>)")
+
+
+@needs_dropin
+@pytest.mark.parametrize("drop_target,remove_every", make_golden.BOOKKEEPING_CASES)
 def test_dropin_bookkeeping_matches_reference(drop_target, remove_every):
     """The drop-in translation units' HOST logic (ldso_b200/host/dropin: insertFrame / insertResidual / dropResidual / removePoint /
     makeIDX, the counters, the connectivity map, hostIDX / targetIDX) against the reference's own EnergyFunctional.cc, both driven through
-    the reference's classes by the same scripted window maintenance (oracle/ref_pin/ref_bench.cc: ref_ba_bookkeeping). No arithmetic member
-    is called: the device context of the drop-in is created lazily, so this runs without a GPU."""
+    the reference's classes by the same scripted window maintenance (oracle/ref_pin/ref_bench.cc: ref_ba_bookkeeping; the reference's
+    record is stored in tests/golden/reference_small.npz). No arithmetic member is called: the device context of the drop-in is created
+    lazily, so this runs without a GPU."""
     import ctypes as C
-    win = synth.make_window(nF=5, pts_per_frame=30, w=320, h=240, seed=5)
-    got = {}
-    for name, lib in (("ref", None), ("dropin", oracle_py.DROPIN_LIB)):
-        r = oracle_py.RefBA(win, multithreaded=False, lib_path=lib)
-        out = (C.c_longlong * 20000)()
-        r.L.ref_ba_bookkeeping.restype = C.c_int
-        n = r.L.ref_ba_bookkeeping(r.o, drop_target, remove_every, out, 20000)
-        assert 0 < n <= 20000
-        got[name] = np.array(out[:n])
+    win = make_golden.ref_window("bookkeeping")
+    got = {"ref": oracle_py.reference_golden()[f"bookkeeping_{drop_target}_{remove_every}"]}
+    r = oracle_py.RefBA(win, multithreaded=False, lib_path=oracle_py.DROPIN_LIB)
+    out = (C.c_longlong * 20000)()
+    r.L.ref_ba_bookkeeping.restype = C.c_int
+    n = r.L.ref_ba_bookkeeping(r.o, drop_target, remove_every, out, 20000)
+    assert 0 < n <= 20000
+    got["dropin"] = np.array(out[:n])
     assert np.array_equal(got["ref"], got["dropin"])
     nF, nP_counter, nR, nAll = got["ref"][:4]
     assert nF == win.nF and nAll == win.nP - (0 if remove_every <= 0 else len(range(0, win.nP, remove_every)))
     assert nR > 0 and (drop_target >= 0 or remove_every > 0 or nR == win.nR)
 
 
-@pytest.mark.skipif(oracle_py.ref_lib() is None or not os.path.exists(oracle_py.DROPIN_LIB),
-                    reason="oracle/_ref/libref_ba.so / libdropin_ba.so are built only where the reference tree is mounted (make -C oracle ref_pin dropin)")
-@pytest.mark.parametrize("geom", [(640, 480, 4, (400.0, 400.0, 319.5, 239.5)), (1232, 368, 5, (718.856, 718.856, 607.1928, 185.2157))])
+@needs_dropin
+@pytest.mark.parametrize("geom", make_golden.MAKE_K_GEOMETRIES)
 def test_dropin_tracker_make_k_matches_reference(geom):
-    """CoarseTracker(w, h) + makeK of the drop-in unit (ldso_b200/host/dropin/dropin_tracker.cc) against the reference's CoarseTracker.cc:
-    the public per-level w, h, fx, fy, cx, cy and inverse intrinsics, bit for bit. Host logic only (the drop-in's device context cannot be
-    created here and says so on stderr; makeK's host side does not depend on it)."""
+    """CoarseTracker(w, h) + makeK of the drop-in unit (ldso_b200/host/dropin/dropin_tracker.cc) against the reference's CoarseTracker.cc
+    (stored in tests/golden/reference_small.npz): the public per-level w, h, fx, fy, cx, cy and inverse intrinsics, bit for bit. Host
+    logic only (the drop-in's device context cannot be created here and says so on stderr; makeK's host side does not depend on it)."""
     import ctypes as C
     w, h, levels, K = geom
     K = np.array(K, np.float64)
-    got = {}
-    for name, lib in (("ref", None), ("dropin", oracle_py.DROPIN_LIB)):
-        L = oracle_py.ref_lib(lib)
-        out = np.zeros(10 * levels)
-        L.ref_tracker_make_k.restype = C.c_int
-        assert L.ref_tracker_make_k(w, h, levels, K.ctypes.data_as(C.POINTER(C.c_double)), out.ctypes.data_as(C.POINTER(C.c_double))) == levels
-        got[name] = out
+    got = {"ref": oracle_py.reference_golden()[f"make_k_{w}x{h}"]}
+    L = oracle_py.ref_lib(oracle_py.DROPIN_LIB)
+    out = np.zeros(10 * levels)
+    L.ref_tracker_make_k.restype = C.c_int
+    assert L.ref_tracker_make_k(w, h, levels, K.ctypes.data_as(C.POINTER(C.c_double)), out.ctypes.data_as(C.POINTER(C.c_double))) == levels
+    got["dropin"] = out
     assert np.array_equal(got["ref"], got["dropin"])
     assert got["ref"][0] == w and got["ref"][10 * (levels - 1)] == w >> (levels - 1)
 
 
 def test_select_activation_golden():
     """The frozen selection case (tests/golden/select_small.npz, written by tests/golden/make_golden.py from the pinned oracle)."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(os.path.dirname(__file__), "golden", "make_golden.py"))
-    mg = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mg)
-    win, newest, args, flagged = mg.select_case()
+    win, newest, args, flagged = make_golden.select_case()
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "select_small.npz"))
     o = oracle_py.OracleBA(win, threads_mode=0)
     for key, dist in (("13", 1.3), ("20", 2.0)):
@@ -453,12 +448,13 @@ def test_select_activation_golden():
     assert np.array_equal(m0.astype(np.uint16), g["map_seed_only"])
 
 
-@pytest.mark.skipif(oracle_py.ref_lib() is None, reason="oracle/_ref/libref_ba.so is built only where the reference tree is mounted")
 def test_reference_tracker_matches_oracle():
-    """The reference's own CoarseTracker::trackNewestCoarse (optimised build in libref_ba.so) and the oracle port find the same pose
-    and brightness on the full-size pair (the bit-exact comparison of the IEEE builds is oracle/ref_pin's)."""
-    pair = synth.make_track_pair()
-    r = oracle_py.RefTracker(pair).track(np.eye(3), np.zeros(3), 0.0, 0.0, pair.levels - 1)
+    """The reference's own CoarseTracker::trackNewestCoarse (optimised build in libref_ba.so, result stored in
+    tests/golden/reference_small.npz) and the oracle port find the same pose and brightness on the full-size pair (the bit-exact
+    comparison of the IEEE builds is oracle/ref_pin's)."""
+    g = oracle_py.reference_golden()
+    pair = make_golden.ref_track_pair("full")
+    r = (bool(g["track_full_ok"]), g["track_full_R"], g["track_full_t"], *g["track_full_aff"])
     o = oracle_py.OracleTracker(pair, fast=True).track(np.eye(3), np.zeros(3), 0.0, 0.0, pair.levels - 1)
     assert r[0] and o[0]
     assert np.abs(r[2] - o[2]).max() < 1e-5 and np.abs(r[1] - o[1]).max() < 1e-5 and abs(r[3] - o[3]) < 1e-4 and abs(r[4] - o[4]) < 1e-2
