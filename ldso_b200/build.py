@@ -36,12 +36,19 @@ def build(force: bool = False, verbose: bool = False) -> str:
         return LIB
     os.makedirs(LIBDIR, exist_ok=True)
     out = os.environ.get("LDSO_B200_LIB", LIB)
-    # trace.cu (immature-point trace) keeps separate multiply/add roundings: its own object, built with -fmad=false
-    trace_o = os.path.join(LIBDIR, "trace.o")
-    base = [f for f in FLAGS if f != "-shared"]
-    subprocess.check_call([NVCC] + base + EXTRA + ["-fmad=false", "-c", os.path.join(CSRC, "trace.cu"), "-o", trace_o])
-    cmd = [NVCC] + FLAGS + EXTRA + (["-Xptxas", "-v"] if verbose else []) + [os.path.join(CSRC, "api.cu"), trace_o, "-o", out]
-    subprocess.check_call(cmd)
+    # one object per .cu unit, compiled side by side; trace.cu (immature-point trace) keeps separate multiply/add roundings:
+    # it is built with -fmad=false
+    base = [f for f in FLAGS if f != "-shared"] + EXTRA + (["-Xptxas", "-v"] if verbose else [])
+    objs, procs = [], []
+    for src in sorted(f for f in os.listdir(CSRC) if f.endswith(".cu")):
+        obj = os.path.join(LIBDIR, src[:-3] + ".o")
+        mad = ["-fmad=false"] if src == "trace.cu" else []
+        procs.append(subprocess.Popen([NVCC] + base + mad + ["-c", os.path.join(CSRC, src), "-o", obj]))
+        objs.append(obj)
+    failed = [p.args for p in procs if p.wait() != 0]
+    if failed:
+        raise subprocess.CalledProcessError(1, failed[0])
+    subprocess.check_call([NVCC] + FLAGS + EXTRA + objs + ["-o", out])
     return out
 
 
